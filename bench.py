@@ -7,12 +7,15 @@ committee, i.e. B x { Mask.SetMask ; Sign.Deserialize ; aggSig.VerifyHash(mask.A
 (reference internal/chain/engine.go:619-642).  `value` counts constituent signatures (set bits) per second with the
 inputs already in HBM; `e2e` is the same metric through the host-buffer C-ABI call (H2D/D2H inside the timed region).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--rounds B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--rounds B] [--impl reference] [--dump-outputs DIR]
 Multi-GPU: torchrun, one rank per GPU; rounds shard by index with no data-path collective (weak scaling).
+--dump-outputs DIR writes the per-round results of the last timed step as DIR/aggregate_verify_results.npy (float32, 1 = the
+round verifies); the inputs are seeded, so two builds can be compared output for output.
 """
 import argparse, ctypes, json, os, subprocess, sys, threading, time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 import numpy as np
 from harmony_b200 import workload as wl
@@ -298,6 +301,21 @@ def other_configs(bls, world, rank, dist, device):
     out["c4_view_change_storm"] = c4
     return out
 
+# ------------------------------------------------------------------ --dump-outputs
+DUMP_MAX_BYTES = 64_000_000
+
+def dump_outputs(out_dir, name, results):
+    """results (uint8 per round) -> out_dir/<name>.npy as float32.  Beyond DUMP_MAX_BYTES a fixed seeded sample of the rounds is
+    written instead, with the sampled round indices beside it in <name>_index.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    res = np.asarray(results, dtype=np.float32)
+    if res.nbytes > DUMP_MAX_BYTES:
+        keep = DUMP_MAX_BYTES // (4 + 8)
+        idx = np.sort(np.random.Generator(np.random.Philox(key=[7, 7])).choice(res.size, size=keep, replace=False))
+        np.save(os.path.join(out_dir, name + "_index.npy"), idx.astype(np.float64))
+        res = res[idx]
+    np.save(os.path.join(out_dir, name + ".npy"), res)
+
 # ------------------------------------------------------------------ main arms
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
@@ -399,6 +417,8 @@ def run_gpu(args):
     launches = bls.KernelLaunchCount() - launches0
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     assert int(d_res.sum().item()) == B
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "aggregate_verify_results" + (f"_rank{rank}" if rank else ""), d_res.cpu().numpy())
     # per-kernel durations: separate passes with event records between the kernels (kept out of the timed region)
     bls.StageTimingEnable(True)
     n_stage = 3; lines_ms = 0.0
@@ -642,7 +662,12 @@ def main():
     ap.add_argument("--rounds", type=int, default=303104, help="rounds per step per GPU (default: 37 888 groups of 8 = one lane pair per group on 148 SMs x 512 threads)")
     ap.add_argument("--impl", default="hbls", choices=["hbls", "reference"])
     ap.add_argument("--no-other-configs", action="store_true", help="skip the short C3 / C4 / C5 legs (BASELINE configs[2..4]) reported beside the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the per-round results of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "hbls":
+        ap.error("--dump-outputs needs --impl hbls")
     if args.warmup < 3 and args.impl == "hbls":
         log("note: warm-up < 3 steps requested")
     if args.impl == "reference":
