@@ -118,6 +118,7 @@ def lib():
         sig("hbls_get_batch_mode", c.c_int)
         sig("hbls_hash_prefetch", c.c_int, u8p, sz)
         sig("hbls_hash_cache_stats", c.c_int, c.POINTER(c.c_uint64), c.POINTER(c.c_uint64))
+        sig("hbls_coalesce_stats", c.c_int, c.POINTER(c.c_uint64), c.POINTER(c.c_uint64), c.POINTER(c.c_uint64))
         sig("hbls_stage_timing_enable", None, c.c_int)
         sig("hbls_stage_timing_get", c.c_int, c.POINTER(c.c_float), c.c_int)
         _lib = L
@@ -366,6 +367,13 @@ def HashCacheStats():
     h = ctypes.c_uint64(0); m = ctypes.c_uint64(0)
     _need().hbls_hash_cache_stats(ctypes.byref(h), ctypes.byref(m))
     return {"hits": h.value, "misses": m.value}
+
+def CoalesceStats():
+    """Coalescing of concurrent per-call operations (VerifyHash, SignHash, Deserialize, GetPublicKey) since the library was loaded:
+    requests queued, batches run, largest batch.  ctypes releases the GIL around each call, so Python threads coalesce too."""
+    r = ctypes.c_uint64(0); b = ctypes.c_uint64(0); m = ctypes.c_uint64(0)
+    _need().hbls_coalesce_stats(ctypes.byref(r), ctypes.byref(b), ctypes.byref(m))
+    return {"requests": r.value, "batches": b.value, "largest_batch": m.value}
 
 def GetPublicKeyBatch(sks32: bytes) -> bytes:
     k = len(sks32) // 32

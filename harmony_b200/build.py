@@ -30,7 +30,7 @@ def _sources(d, exts):
 
 def build_cuda(force=False, verbose=False):
     os.makedirs(LIBDIR, exist_ok=True)
-    srcs = _sources(CSRC, (".cu", ".cuh", ".h")) + [os.path.join(ROOT, "include", "hbls.h")]
+    srcs = _sources(CSRC, (".cu", ".cuh", ".h", ".hpp")) + [os.path.join(ROOT, "include", "hbls.h")]
     if not force and _newer(LIB, srcs):
         return LIB
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

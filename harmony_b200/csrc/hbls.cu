@@ -9,8 +9,11 @@
 #include <map>
 #include <memory>
 #include <mutex>
+#include <string>
+#include <unordered_map>
 #include <vector>
 #include "../../include/hbls.h"
+#include "coalesce.hpp"
 #include "kernels.cuh"
 
 using namespace hb;
@@ -56,6 +59,8 @@ struct Ctx {
     g2a* hm_slots = nullptr; uint8_t* hm_ok = nullptr; HmEntry hm[HM_N];
     uint64_t hm_clock = 0, hm_hits = 0, hm_misses = 0;
     long long hm_cache = 1;                                 // hbls_set_param("hm_cache", 0) turns it off (cold-path measurements)
+    // pinned host staging of the per-call operations (device -> host copies of a coalesced batch, hbls.cu co_run)
+    uint8_t* pin = nullptr; size_t pin_cap = 0;
 };
 Ctx g;
 
@@ -102,6 +107,18 @@ int reserve(cudaStream_t s, size_t bytes, Scratch** out) {
     return 0;
 }
 inline unsigned blocks_for(size_t n, unsigned tpb) { return (unsigned)((n + tpb - 1) / tpb); }
+// pinned host staging of at least `bytes` (growing frees the old block: callers hold g.mu and have synchronised their copies)
+int reserve_pinned(size_t bytes, uint8_t** out) {
+    if (bytes > g.pin_cap) {
+        if (g.pin) CK(cudaFreeHost(g.pin));
+        g.pin = nullptr; g.pin_cap = 0;
+        const size_t cap = bytes + bytes / 4 + 4096;
+        CK(cudaMallocHost(&g.pin, cap));
+        g.pin_cap = cap;
+    }
+    *out = g.pin;
+    return 0;
+}
 
 // ------------------------------------------------------------------ H(m) cache.  Caller holds g.mu.  Entries are filled and read on
 // whatever stream the call runs on; `filled` orders readers after the fill, `read_done` orders a later overwrite after the readers.
@@ -456,7 +473,7 @@ int single_op(int op, const void* a, size_t an, const void* b, size_t bn, void* 
     int rc = 0;
     CK(cudaMemcpyAsync(&rc, drc, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
     CK(cudaStreamSynchronize(g.stream));
-    if (on && rc >= 0 && !((op == OP_G1_DES || op == OP_G2_DES) && rc == 0) && !(op == OP_MAP_SER && rc != 0))
+    if (on && rc >= 0 && !(op == OP_MAP_SER && rc != 0))
         CK(cudaMemcpy(out, dout, on, cudaMemcpyDeviceToHost));
     *rc_out = rc;
     return 0;
@@ -770,10 +787,6 @@ size_t blsPublicKeySerialize(void* buf, size_t maxBufSize, const blsPublicKey* p
     if (maxBufSize < 48) return 0; int rc = 0; if (single_op(OP_G1_SER, pub, 144, nullptr, 0, buf, 48, &rc)) return 0; return rc == 48 ? 48 : 0; }
 size_t blsSignatureSerialize(void* buf, size_t maxBufSize, const blsSignature* sig) {
     if (maxBufSize < 96) return 0; int rc = 0; if (single_op(OP_G2_SER, sig, 288, nullptr, 0, buf, 96, &rc)) return 0; return rc == 96 ? 96 : 0; }
-size_t blsPublicKeyDeserialize(blsPublicKey* pub, const void* buf, size_t bufSize) {
-    if (bufSize < 48) return 0; int rc = 0; if (single_op(OP_G1_DES, buf, 48, nullptr, 0, pub, 144, &rc)) return 0; return rc == 48 ? 48 : 0; }
-size_t blsSignatureDeserialize(blsSignature* sig, const void* buf, size_t bufSize) {
-    if (bufSize < 96) return 0; int rc = 0; if (single_op(OP_G2_DES, buf, 96, nullptr, 0, sig, 288, &rc)) return 0; return rc == 96 ? 96 : 0; }
 int hbls_map_to_g2(const void* msg, size_t msg_len, uint8_t out96[96]) {
     if (msg_len > 48) msg_len = 48;      // only the first 48 bytes matter (SURVEY A.3)
     int rc = -1; if (int e = single_op(OP_MAP_SER, msg, msg_len, nullptr, 0, out96, 96, &rc, (uint32_t)msg_len)) return e; return rc; }
@@ -809,93 +822,246 @@ int hbls_get_address(const blsPublicKey* pub, uint8_t out20[20]) {
     Sha256::digest(ser, 48, dg); memcpy(out20, dg, 20); return 0;
 }
 
-void blsGetPublicKey(blsPublicKey* pub, const blsSecretKey* sec) {
-    memset(pub, 0, sizeof *pub);
-    if (ensure_init()) return;
-    std::lock_guard<std::mutex> lk(g.mu);
-    Scratch* sc; if (reserve(g.stream, 4096, &sc)) return;
-    Arena ar{sc->base, 0, sc->cap};
-    uint8_t* dsk = ar.take<uint8_t>(32); g1* dout = ar.take<g1>(1);
-    blsPublicKey tmp;
-    cudaError_t e = cudaMemcpyAsync(dsk, sec->d, 32, cudaMemcpyHostToDevice, g.stream);
-    LAUNCH(k_g1_mul_gen, 1, 32, g.stream, (size_t)1, dsk, dout);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&tmp, dout, 144, cudaMemcpyDeviceToHost, g.stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(g.stream);
-    if (e != cudaSuccess) { note_error(e, "blsGetPublicKey", __FILE__, __LINE__); return; }
-    *pub = tmp;
-}
-int blsSignHash(blsSignature* sig, const blsSecretKey* sec, const void* h, size_t size) {
-    if (int e = ensure_init()) return e;
-    std::lock_guard<std::mutex> lk(g.mu);
-    if (size > 48) size = 48;
-    Scratch* sc; if (int e = reserve(g.stream, 4096, &sc)) return e;
-    Arena ar{sc->base, 0, sc->cap};
-    uint8_t* dsk = ar.take<uint8_t>(32); uint8_t* dmsg = ar.take<uint8_t>(64); g2* dout = ar.take<g2>(1); uint8_t* dok = ar.take<uint8_t>(1);
-    g2a* dhm = ar.take<g2a>(1); uint8_t* dhm_ok = ar.take<uint8_t>(1);
-    CK(cudaMemcpyAsync(dsk, sec->d, 32, cudaMemcpyHostToDevice, g.stream));
-    if (size) CK(cudaMemcpyAsync(dmsg, h, size, cudaMemcpyHostToDevice, g.stream));
-    // H(m) on a lane pair (kept in the H(m) cache: the validator verifies the aggregate over the very message it signs here), then
-    // the 255-bit ladder sk * H on the split carrier
-    uint8_t key[48]; bool hit = false;
-    if (hm_enabled()) { hm_key(key, h, size); hit = hm_fetch(key, dhm, dhm_ok, g.stream); }
-    if (!hit) {
-        launch_hash_small(g.stream, 1, dmsg, (uint32_t)size, dhm, dhm_ok);
-        if (hm_enabled()) hm_store(key, dhm, dhm_ok, g.stream);
+}  // extern "C"
+
+// ------------------------------------------------------------------ per-call operations, coalesced (coalesce.hpp).  Concurrent
+// VerifyHash / SignHash / Deserialize / GetPublicKey calls queue up; one caller at a time takes g.mu, drains the queue and runs ONE
+// batched device pass per operation kind over everything drained, with one stream synchronise.  A batch of one is the single call.
+namespace {
+
+struct HashMsg { const void* h; size_t size; };
+// device bytes of launch_hm_batch over k items (every take of the arena is 256-byte aligned)
+size_t hm_batch_bytes(size_t k) { return k * (sizeof(g2a) + 1 + 48 + 4) + 8 * 256; }
+// H(m) of k items into hm / ok, each DISTINCT message once: the distinct messages (keyed by the 48 zero-padded bytes hash_to_fp reads,
+// hm_key) are looked up in the H(m) cache, the misses are hashed in one launch and stored, then k_hm_gather copies every item's point
+// from the distinct array.  Cache hit / miss counters count distinct messages.  Caller holds g.mu; runs on g.stream.
+int launch_hm_batch(Arena& ar, size_t k, const HashMsg* msgs, g2a* hm, uint8_t* ok) {
+    const bool cache = hm_enabled();
+    std::vector<uint8_t> ukey(48 * k); std::vector<uint32_t> item_u(k);
+    std::unordered_map<std::string, uint32_t> seen; seen.reserve(2 * k);
+    size_t nu = 0;
+    for (size_t i = 0; i < k; i++) {
+        uint8_t key[48]; hm_key(key, msgs[i].h, msgs[i].size);
+        auto ins = seen.emplace(std::string((const char*)key, 48), (uint32_t)nu);
+        if (ins.second) memcpy(&ukey[48 * nu++], key, 48);
+        item_u[i] = ins.first->second;
     }
-    // sk in base |z| (four 64-bit digits): the ladder runs over psi (kernels.cuh k_sign_hm_gls_pair)
-    uint64_t dig[4];
-    if (sk_digits_base_z(sec->d, dig)) {
-        uint64_t* ddig = ar.take<uint64_t>(4);
-        CK(cudaMemcpyAsync(ddig, dig, sizeof dig, cudaMemcpyHostToDevice, g.stream));
-        LAUNCH(k_sign_hm_gls_pair, 1, 32, g.stream, (size_t)1, ddig, dhm, dhm_ok, (size_t)0, dout, dok);
-    } else
-        LAUNCH(k_sign_hm_pair, 1, 32, g.stream, (size_t)1, dsk, dhm, dhm_ok, (size_t)0, dout, dok);
-    uint8_t ok = 0;
-    CK(cudaMemcpyAsync(sig, dout, 288, cudaMemcpyDeviceToHost, g.stream));
-    CK(cudaMemcpyAsync(&ok, dok, 1, cudaMemcpyDeviceToHost, g.stream));
-    CK(cudaStreamSynchronize(g.stream));
-    return ok ? 0 : -1;
+    g2a* dhm = ar.take<g2a>(nu); uint8_t* dok = ar.take<uint8_t>(nu); uint8_t* dkeys = ar.take<uint8_t>(48 * nu); uint32_t* didx = ar.take<uint32_t>(k);
+    // slots of the distinct array: misses from the front (one contiguous hash launch), cache hits from the back
+    std::vector<uint32_t> slot(nu); std::vector<uint8_t> mkeys; mkeys.reserve(48 * nu);
+    size_t lo = 0, hi = nu;
+    for (size_t u = 0; u < nu; u++) {
+        if (cache && hm_fetch(&ukey[48 * u], dhm + hi - 1, dok + hi - 1, g.stream)) slot[u] = (uint32_t)--hi;
+        else { slot[u] = (uint32_t)lo++; mkeys.insert(mkeys.end(), &ukey[48 * u], &ukey[48 * u] + 48); }
+    }
+    if (lo) {
+        CK(cudaMemcpyAsync(dkeys, mkeys.data(), 48 * lo, cudaMemcpyHostToDevice, g.stream));
+        launch_hash_small(g.stream, lo, dkeys, 48, dhm, dok);
+        if (cache)                                   // only the last HM_N would survive anyway
+            for (size_t j = lo > (size_t)Ctx::HM_N ? lo - Ctx::HM_N : 0; j < lo; j++) hm_store(&mkeys[48 * j], dhm + j, dok + j, g.stream);
+    }
+    std::vector<uint32_t> idx(k);
+    for (size_t i = 0; i < k; i++) idx[i] = slot[item_u[i]];
+    CK(cudaMemcpyAsync(didx, idx.data(), 4 * k, cudaMemcpyHostToDevice, g.stream));
+    LAUNCH(k_hm_gather, blocks_for(k, 128), 128, g.stream, k, (const uint32_t*)didx, (const g2a*)dhm, (const uint8_t*)dok, hm, ok);
+    return 0;
 }
-// VerifyHash on already-decoded structs: d_apk (device Jacobian key) or host pub; returns 1 / 0, <0 on error.  Caller holds g.mu.
-static int verify_hash_locked(const blsSignature* sig, const blsPublicKey* pub, const g1* d_apk, const uint8_t* sig96, const void* h, size_t size) {
-    if (size > 48) size = 48;
-    Scratch* sc; if (int e = reserve(g.stream, verify_scratch_bytes(1) + 4096, &sc)) return e;
-    Arena ar{sc->base, 0, sc->cap};
-    VerifyBufs v = carve_verify(ar, 1);
-    g2* dsig = ar.take<g2>(1); uint8_t* dsig96 = ar.take<uint8_t>(96); uint8_t* dmsg = ar.take<uint8_t>(64); uint8_t* dres = ar.take<uint8_t>(1);
-    if (d_apk) CK(cudaMemcpyAsync(v.apk, d_apk, 144, cudaMemcpyDeviceToDevice, g.stream));
-    else CK(cudaMemcpyAsync(v.apk, pub, 144, cudaMemcpyHostToDevice, g.stream));
-    if (size) CK(cudaMemcpyAsync(dmsg, h, size, cudaMemcpyHostToDevice, g.stream));
-    LAUNCH(k_g1_normalize_lat, 1, 32, g.stream, (size_t)1, v.apk, v.pkneg, 1);
+
+size_t verify_pass_bytes(size_t k) { return verify_scratch_bytes(k) + k * (sizeof(g2) + 1) + 96 + hm_batch_bytes(k) + 16 * 256; }
+// VerifyHash of k items, enqueued on g.stream; res[j] (pinned host) is valid once the stream has synchronised.  Keys: host structs
+// (pubs) or one device Jacobian key (d_apk, k = 1: hbls_mask_verify); signatures: host structs (sigs) or one serialized signature
+// (sig96, k = 1), decoded and subgroup-checked on the device.  Caller holds g.mu and reserved verify_pass_bytes(k).
+int verify_hash_locked(Arena& ar, size_t k, const blsSignature* const* sigs, const uint8_t* sig96, const blsPublicKey* const* pubs,
+                       const g1* d_apk, const HashMsg* msgs, uint8_t* res) {
+    VerifyBufs v = carve_verify(ar, k);
+    g2* dsig = ar.take<g2>(k); uint8_t* dsig96 = ar.take<uint8_t>(96); uint8_t* dres = ar.take<uint8_t>(k);
+    if (d_apk) CK(cudaMemcpyAsync(v.apk, d_apk, sizeof(g1), cudaMemcpyDeviceToDevice, g.stream));
+    else {
+        std::vector<g1> hp(k);
+        for (size_t j = 0; j < k; j++) memcpy(&hp[j], pubs[j], sizeof(g1));
+        CK(cudaMemcpyAsync(v.apk, hp.data(), k * sizeof(g1), cudaMemcpyHostToDevice, g.stream));
+    }
+    LAUNCH(k_g1_normalize_lat, blocks_for(k, 32), 32, g.stream, k, v.apk, v.pkneg, 1);
     const uint8_t* ok_sig = nullptr;
     if (sig96) {          // serialized signature: decode (+ subgroup check) on the device
         CK(cudaMemcpyAsync(dsig96, sig96, 96, cudaMemcpyHostToDevice, g.stream));
-        LAUNCH(k_g2_decode_pair, 1, 32, g.stream, (size_t)1, dsig96, v.sig, v.ok_sig, 1);
+        LAUNCH(k_g2_decode_pair, 1, 32, g.stream, (size_t)1, dsig96, v.sig, v.ok_sig, 1, (g2*)nullptr);
         ok_sig = v.ok_sig;
     } else {              // struct inputs are already-decoded Jacobian points: normalise instead of decoding
-        CK(cudaMemcpyAsync(dsig, sig, 288, cudaMemcpyHostToDevice, g.stream));
-        LAUNCH(k_g2_normalize, 1, 32, g.stream, (size_t)1, dsig, v.sig);
+        std::vector<g2> hs(k);
+        for (size_t j = 0; j < k; j++) memcpy(&hs[j], sigs[j], sizeof(g2));
+        CK(cudaMemcpyAsync(dsig, hs.data(), k * sizeof(g2), cudaMemcpyHostToDevice, g.stream));
+        LAUNCH(k_g2_normalize, blocks_for(k, 32), 32, g.stream, k, dsig, v.sig);
     }
-    {   // H(m): cached when this node has hashed the message before (its own SignHash, a prefetch, an earlier check)
-        uint8_t key[48]; bool hit = false;
-        if (hm_enabled()) { hm_key(key, h, size); hit = hm_fetch(key, v.hm, v.ok_hm, g.stream); }
-        if (!hit) {
-            launch_hash_small(g.stream, 1, dmsg, (uint32_t)size, v.hm, v.ok_hm);
-            if (hm_enabled()) hm_store(key, v.hm, v.ok_hm, g.stream);
-        }
+    // H(m): cached when this node has hashed the message before (its own SignHash, a prefetch, an earlier check)
+    if (int e = launch_hm_batch(ar, k, msgs, v.hm, v.ok_hm)) return e;
+    if ((long long)k <= g.coop_max) {       // one warp per check
+        const size_t coop_cap = (size_t)g.sm_count * (size_t)(g.coop_wpsm > 0 ? g.coop_wpsm : 1);
+        LAUNCH(k_pairing_coop, (unsigned)(k < coop_cap ? k : coop_cap), 32, g.stream, k, v.sig, v.pkneg, v.hm, (const uint8_t*)v.ok_hm, ok_sig, (const uint8_t*)nullptr, dres);
+    } else
+        LAUNCH(k_pairing_verify_split, blocks_for(2 * k, 64), 64, g.stream, k, v.sig, v.pkneg, v.hm, (const uint8_t*)v.ok_hm, ok_sig, (const uint8_t*)nullptr, dres, (const int*)nullptr);
+    LAUNCH(k_pairing_fixup, heavy_blocks(k), TPB, g.stream, k, v.sig, v.pkneg, v.hm, (const uint8_t*)v.ok_hm, ok_sig, (const uint8_t*)nullptr, dres, (const int*)nullptr);
+    CK(cudaMemcpyAsync(res, dres, k, cudaMemcpyDeviceToHost, g.stream));
+    return 0;
+}
+
+enum CoOp { CO_VERIFY, CO_SIGN, CO_SIG_DES, CO_PK_DES, CO_GET_PK, CO_NOPS };
+// one queued per-call request: a = signature struct (verify) / secret key (sign, get-pk) / serialized bytes (deserialize),
+// b = public key struct (verify), out = the caller's struct; rc = the call's result, written by the combiner
+struct CoReq { int op; const void* a; const void* b; const void* msg; size_t len; void* out; int rc; };
+hb::FlatCombiner<CoReq> g_co;
+
+size_t sign_pass_bytes(size_t k) { return k * (32 + 32 + sizeof(g2) + 1 + sizeof(g2a) + 1) + 2 * hm_batch_bytes(k) + 16 * 256; }
+// SignHash of k items (sigma = sk H(m)): into h_out / h_ok (pinned host) at position p for item perm[p].  Keys with base-|z| digits
+// (every sk < r) take the ladder over psi; hand-filled structs >= Z^4 a second sub-batch through the plain 255-bit ladder.
+int launch_sign_pass(Arena& ar, const std::vector<CoReq*>& rq, g2* h_out, uint8_t* h_ok, std::vector<uint32_t>& perm) {
+    const size_t k = rq.size();
+    std::vector<uint64_t> dig; std::vector<uint8_t> sk; std::vector<uint32_t> ib; std::vector<HashMsg> ma, mb;
+    perm.clear();
+    for (size_t j = 0; j < k; j++) {
+        const blsSecretKey* sec = (const blsSecretKey*)rq[j]->a; uint64_t d[4];
+        const HashMsg m{rq[j]->msg, rq[j]->len};
+        if (sk_digits_base_z(sec->d, d)) { dig.insert(dig.end(), d, d + 4); perm.push_back((uint32_t)j); ma.push_back(m); }
+        else { sk.insert(sk.end(), (const uint8_t*)sec->d, (const uint8_t*)sec->d + 32); ib.push_back((uint32_t)j); mb.push_back(m); }
     }
-    if (g.coop_max >= 1) LAUNCH(k_pairing_coop, 1, 32, g.stream, (size_t)1, v.sig, v.pkneg, v.hm, (const uint8_t*)v.ok_hm, ok_sig, (const uint8_t*)nullptr, dres);
-    else LAUNCH(k_pairing_verify_split, 1, 64, g.stream, (size_t)1, v.sig, v.pkneg, v.hm, (const uint8_t*)v.ok_hm, ok_sig, (const uint8_t*)nullptr, dres, (const int*)nullptr);
-    LAUNCH(k_pairing_fixup, 1, 32, g.stream, (size_t)1, v.sig, v.pkneg, v.hm, (const uint8_t*)v.ok_hm, ok_sig, (const uint8_t*)nullptr, dres, (const int*)nullptr);
-    uint8_t res = 0;
-    CK(cudaMemcpyAsync(&res, dres, 1, cudaMemcpyDeviceToHost, g.stream));
+    const size_t na = ma.size(), nb = mb.size();
+    perm.insert(perm.end(), ib.begin(), ib.end());
+    g2* dout = ar.take<g2>(k); uint8_t* dok = ar.take<uint8_t>(k);
+    g2a* hm = ar.take<g2a>(k); uint8_t* hok = ar.take<uint8_t>(k);
+    if (na) {
+        uint64_t* ddig = ar.take<uint64_t>(4 * na);
+        CK(cudaMemcpyAsync(ddig, dig.data(), 32 * na, cudaMemcpyHostToDevice, g.stream));
+        if (int e = launch_hm_batch(ar, na, ma.data(), hm, hok)) return e;
+        LAUNCH(k_sign_hm_gls_pair, blocks_for(2 * na, 32), 32, g.stream, na, (const uint64_t*)ddig, (const g2a*)hm, (const uint8_t*)hok, (size_t)1, dout, dok);
+    }
+    if (nb) {
+        uint8_t* dsk = ar.take<uint8_t>(32 * nb);
+        CK(cudaMemcpyAsync(dsk, sk.data(), 32 * nb, cudaMemcpyHostToDevice, g.stream));
+        if (int e = launch_hm_batch(ar, nb, mb.data(), hm + na, hok + na)) return e;
+        LAUNCH(k_sign_hm_pair, blocks_for(2 * nb, 32), 32, g.stream, nb, (const uint8_t*)dsk, (const g2a*)(hm + na), (const uint8_t*)(hok + na), (size_t)1, dout + na, dok + na);
+    }
+    CK(cudaMemcpyAsync(h_out, dout, k * sizeof(g2), cudaMemcpyDeviceToHost, g.stream));
+    CK(cudaMemcpyAsync(h_ok, dok, k, cudaMemcpyDeviceToHost, g.stream));
+    return 0;
+}
+
+// one device pass per operation kind present, one synchronise, then every caller's output and return value.  g.mu is held.
+int co_launch(const std::vector<CoReq*>* by) {
+    const size_t kv = by[CO_VERIFY].size(), ks = by[CO_SIGN].size(), kd2 = by[CO_SIG_DES].size(), kd1 = by[CO_PK_DES].size(), kg = by[CO_GET_PK].size();
+    size_t dev = 4096, host = 8 * 256;
+    if (kv) { dev += verify_pass_bytes(kv); host += kv + 256; }
+    if (ks) { dev += sign_pass_bytes(ks); host += ks * (sizeof(g2) + 1) + 512; }
+    if (kd2) { dev += kd2 * (96 + sizeof(g2) + 1) + 4 * 256; host += kd2 * (sizeof(g2) + 1) + 512; }
+    if (kd1) { dev += kd1 * (48 + sizeof(g1) + 1) + 4 * 256; host += kd1 * (sizeof(g1) + 1) + 512; }
+    if (kg) { dev += kg * (32 + sizeof(g1)) + 4 * 256; host += kg * sizeof(g1) + 512; }
+    Scratch* sc; if (int e = reserve(g.stream, dev, &sc)) return e;
+    uint8_t* pin; if (int e = reserve_pinned(host, &pin)) return e;
+    Arena ar{sc->base, 0, sc->cap}, hp{pin, 0, g.pin_cap};
+    uint8_t* v_res = nullptr; g2* s_out = nullptr; uint8_t* s_ok = nullptr; std::vector<uint32_t> s_perm;
+    g2* d2_out = nullptr; uint8_t* d2_ok = nullptr; g1* d1_out = nullptr; uint8_t* d1_ok = nullptr; g1* pk_out = nullptr;
+    if (kv) {
+        std::vector<const blsSignature*> sigs(kv); std::vector<const blsPublicKey*> pubs(kv); std::vector<HashMsg> msgs(kv);
+        for (size_t j = 0; j < kv; j++) { const CoReq* r = by[CO_VERIFY][j]; sigs[j] = (const blsSignature*)r->a; pubs[j] = (const blsPublicKey*)r->b; msgs[j] = {r->msg, r->len}; }
+        v_res = hp.take<uint8_t>(kv);
+        if (int e = verify_hash_locked(ar, kv, sigs.data(), nullptr, pubs.data(), nullptr, msgs.data(), v_res)) return e;
+    }
+    if (ks) {
+        s_out = hp.take<g2>(ks); s_ok = hp.take<uint8_t>(ks);
+        if (int e = launch_sign_pass(ar, by[CO_SIGN], s_out, s_ok, s_perm)) return e;
+    }
+    if (kd2) {            // Sign.Deserialize: lane-pair decode + subgroup test, written in the blsSignature layout
+        std::vector<uint8_t> in(96 * kd2);
+        for (size_t j = 0; j < kd2; j++) memcpy(&in[96 * j], by[CO_SIG_DES][j]->a, 96);
+        uint8_t* din = ar.take<uint8_t>(96 * kd2); g2* dout = ar.take<g2>(kd2); uint8_t* dok = ar.take<uint8_t>(kd2);
+        d2_out = hp.take<g2>(kd2); d2_ok = hp.take<uint8_t>(kd2);
+        CK(cudaMemcpyAsync(din, in.data(), 96 * kd2, cudaMemcpyHostToDevice, g.stream));
+        LAUNCH(k_g2_decode_pair, blocks_for(2 * kd2, 32), 32, g.stream, kd2, (const uint8_t*)din, (g2a*)nullptr, dok, 1, dout);
+        CK(cudaMemcpyAsync(d2_out, dout, kd2 * sizeof(g2), cudaMemcpyDeviceToHost, g.stream));
+        CK(cudaMemcpyAsync(d2_ok, dok, kd2, cudaMemcpyDeviceToHost, g.stream));
+    }
+    if (kd1) {            // PublicKey.Deserialize: decode + subgroup test, Jacobian with z = 1 (the blsPublicKey layout)
+        std::vector<uint8_t> in(48 * kd1);
+        for (size_t j = 0; j < kd1; j++) memcpy(&in[48 * j], by[CO_PK_DES][j]->a, 48);
+        uint8_t* din = ar.take<uint8_t>(48 * kd1); g1* dout = ar.take<g1>(kd1); uint8_t* dok = ar.take<uint8_t>(kd1);
+        d1_out = hp.take<g1>(kd1); d1_ok = hp.take<uint8_t>(kd1);
+        CK(cudaMemcpyAsync(din, in.data(), 48 * kd1, cudaMemcpyHostToDevice, g.stream));
+        LAUNCH(k_g1_decode_jac, heavy_blocks(kd1), TPB, g.stream, kd1, (const uint8_t*)din, dout, dok, 1);
+        CK(cudaMemcpyAsync(d1_out, dout, kd1 * sizeof(g1), cudaMemcpyDeviceToHost, g.stream));
+        CK(cudaMemcpyAsync(d1_ok, dok, kd1, cudaMemcpyDeviceToHost, g.stream));
+    }
+    if (kg) {             // GetPublicKey: sk * generator
+        std::vector<uint8_t> sk(32 * kg);
+        for (size_t j = 0; j < kg; j++) memcpy(&sk[32 * j], ((const blsSecretKey*)by[CO_GET_PK][j]->a)->d, 32);
+        uint8_t* dsk = ar.take<uint8_t>(32 * kg); g1* dout = ar.take<g1>(kg);
+        pk_out = hp.take<g1>(kg);
+        CK(cudaMemcpyAsync(dsk, sk.data(), 32 * kg, cudaMemcpyHostToDevice, g.stream));
+        LAUNCH(k_g1_mul_gen, blocks_for(kg, 32), 32, g.stream, kg, (const uint8_t*)dsk, dout);
+        CK(cudaMemcpyAsync(pk_out, dout, kg * sizeof(g1), cudaMemcpyDeviceToHost, g.stream));
+    }
     CK(cudaStreamSynchronize(g.stream));
-    return res ? 1 : 0;
+    for (size_t j = 0; j < kv; j++) by[CO_VERIFY][j]->rc = v_res[j] ? 1 : 0;
+    for (size_t p = 0; p < ks; p++) {
+        CoReq* r = by[CO_SIGN][s_perm[p]];
+        memcpy(r->out, &s_out[p], sizeof(g2)); r->rc = s_ok[p] ? 0 : -1;
+    }
+    for (size_t j = 0; j < kd2; j++) {            // undecodable: the caller's struct stays as it was
+        CoReq* r = by[CO_SIG_DES][j];
+        if (d2_ok[j]) memcpy(r->out, &d2_out[j], sizeof(g2));
+        r->rc = d2_ok[j] ? 96 : 0;
+    }
+    for (size_t j = 0; j < kd1; j++) {
+        CoReq* r = by[CO_PK_DES][j];
+        if (d1_ok[j]) memcpy(r->out, &d1_out[j], sizeof(g1));
+        r->rc = d1_ok[j] ? 48 : 0;
+    }
+    for (size_t j = 0; j < kg; j++) { memcpy(by[CO_GET_PK][j]->out, &pk_out[j], sizeof(g1)); by[CO_GET_PK][j]->rc = 0; }
+    return 0;
+}
+void co_run(CoReq* const* batch, size_t n) {
+    std::vector<CoReq*> by[CO_NOPS];
+    for (size_t i = 0; i < n; i++) by[batch[i]->op].push_back(batch[i]);
+    int e;
+    try { e = co_launch(by); } catch (const std::exception&) { e = HBLS_ERR_CUDA; }      // (bad_alloc) the owners must still be woken
+    if (e) for (size_t i = 0; i < n; i++) batch[i]->rc = e;
+}
+int co_submit(int op, const void* a, const void* b, const void* msg, size_t len, void* out) {
+    CoReq r{op, a, b, msg, len, out, 0};
+    g_co.submit(r, g.mu, [] { return g.coop_max; }, co_run);
+    return r.rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+void blsGetPublicKey(blsPublicKey* pub, const blsSecretKey* sec) {
+    memset(pub, 0, sizeof *pub);
+    if (ensure_init()) return;
+    co_submit(CO_GET_PK, sec, nullptr, nullptr, 0, pub);
+}
+int blsSignHash(blsSignature* sig, const blsSecretKey* sec, const void* h, size_t size) {
+    if (int e = ensure_init()) return e;
+    // H(m) kept in the H(m) cache: the validator verifies the aggregate over the very message it signs here
+    return co_submit(CO_SIGN, sec, nullptr, h, size, sig);
 }
 int blsVerifyHash(const blsSignature* sig, const blsPublicKey* pub, const void* h, size_t size) {
     if (ensure_init()) return 0;
-    std::lock_guard<std::mutex> lk(g.mu);
-    return verify_hash_locked(sig, pub, nullptr, nullptr, h, size) == 1 ? 1 : 0;
+    return co_submit(CO_VERIFY, sig, pub, h, size, nullptr) == 1 ? 1 : 0;
+}
+size_t blsPublicKeyDeserialize(blsPublicKey* pub, const void* buf, size_t bufSize) {
+    if (bufSize < 48 || ensure_init()) return 0;
+    return co_submit(CO_PK_DES, buf, nullptr, nullptr, 0, pub) == 48 ? 48 : 0;
+}
+size_t blsSignatureDeserialize(blsSignature* sig, const void* buf, size_t bufSize) {
+    if (bufSize < 96 || ensure_init()) return 0;
+    return co_submit(CO_SIG_DES, buf, nullptr, nullptr, 0, sig) == 96 ? 96 : 0;
+}
+int hbls_coalesce_stats(uint64_t* requests, uint64_t* batches, uint64_t* largest_batch) {
+    const hb::CoalesceStats s = g_co.stats();
+    if (requests) *requests = s.requests;
+    if (batches) *batches = s.batches;
+    if (largest_batch) *largest_batch = s.largest_batch;
+    return 0;
 }
 void blsSign(blsSignature* sig, const blsSecretKey* sec, const void* m, size_t size) {
     uint8_t dg[64]; Sha512::digest((const uint8_t*)m, size, dg);
@@ -1135,10 +1301,8 @@ int hbls_mask_clear(hbls_mask* m) {
     CK(cudaStreamSynchronize(g.stream));
     return 0;
 }
-int hbls_mask_set_mask(hbls_mask* m, const uint8_t* bitmap, size_t blen) {
-    if (int e = ensure_init()) return e;
-    if (!m || blen != m->bitmap.size()) return HBLS_ERR_ARG;          // mask.go:114-120 "mismatching bitmap lengths"
-    std::lock_guard<std::mutex> lk(g.mu);
+// SetMask body (caller holds g.mu): apply the delta between m's bitmap and `bitmap` to the running aggregate key
+static int set_mask_locked(hbls_mask* m, const uint8_t* bitmap, size_t blen) {
     const size_t n = m->c->n;
     std::vector<uint8_t> delta(2 * blen + 2, 0);                       // row 0: bits to Add (0 -> 1), row 1: bits to Sub (1 -> 0)
     bool any = false;
@@ -1162,13 +1326,21 @@ int hbls_mask_set_mask(hbls_mask* m, const uint8_t* bitmap, size_t blen) {
     }
     return 0;
 }
+int hbls_mask_set_mask(hbls_mask* m, const uint8_t* bitmap, size_t blen) {
+    if (int e = ensure_init()) return e;
+    if (!m || blen != m->bitmap.size()) return HBLS_ERR_ARG;          // mask.go:114-120 "mismatching bitmap lengths"
+    std::lock_guard<std::mutex> lk(g.mu);
+    return set_mask_locked(m, bitmap, blen);
+}
 int hbls_mask_set_bit(hbls_mask* m, size_t index, int enable) {
+    if (int e = ensure_init()) return e;
     if (!m || index >= m->c->n) return HBLS_ERR_ARG;                   // mask.go:138-140 "index out of range"
-    std::vector<uint8_t> bm;
-    { std::lock_guard<std::mutex> lk(g.mu); bm = m->bitmap; }
+    // read-modify-write of the bitmap under ONE hold of g.mu: concurrent SetBit calls on different bits all land
+    std::lock_guard<std::mutex> lk(g.mu);
+    std::vector<uint8_t> bm = m->bitmap;
     const uint8_t msk = (uint8_t)(1u << (index & 7));
     if (enable) bm[index >> 3] |= msk; else bm[index >> 3] &= (uint8_t)~msk;
-    return hbls_mask_set_mask(m, bm.data(), bm.size());
+    return set_mask_locked(m, bm.data(), bm.size());
 }
 int hbls_mask_count_enabled(const hbls_mask* m) {
     if (!m) return HBLS_ERR_ARG;
@@ -1194,7 +1366,13 @@ int hbls_mask_verify(const hbls_mask* m, const uint8_t sig96[96], const void* ms
     if (int e = ensure_init()) return e;
     if (!m || !sig96) return HBLS_ERR_ARG;
     std::lock_guard<std::mutex> lk(g.mu);
-    return verify_hash_locked(nullptr, nullptr, m->d_acc, sig96, msg, msg_len);
+    Scratch* sc; if (int e = reserve(g.stream, verify_pass_bytes(1), &sc)) return e;
+    uint8_t* res; if (int e = reserve_pinned(1, &res)) return e;
+    Arena ar{sc->base, 0, sc->cap};
+    const HashMsg hm{msg, msg_len};
+    if (int e = verify_hash_locked(ar, 1, nullptr, sig96, nullptr, m->d_acc, &hm, res)) return e;
+    CK(cudaStreamSynchronize(g.stream));
+    return res[0] ? 1 : 0;
 }
 int hbls_ballot_box_create(hbls_ballot_box** out, const hbls_committee* c) {
     if (int e = ensure_init()) return e;

@@ -353,7 +353,10 @@ __global__ void k_hash_cofactor(size_t n, g2a* pts, const uint8_t* ok) {
 // ---- lane-pair forms of decode / hash for small batches (latency path, hbls.cu: B <= coop_max): one item per LANE PAIR.  The Fp-only
 // chains (square roots, Jacobi symbols, the SW map) run redundantly on both lanes; the long G2 ladders -- subgroup test, cofactor
 // clearing -- run on the split carrier (an Fp2 product costs one product-time per lane instead of three), inversions by binary GCD.
-__global__ void k_g2_decode_pair(size_t n, const uint8_t* in, g2a* out, uint8_t* ok, int check_order) {
+// out_jac (nullable): the decoded point is ALSO written in the blsSignature layout -- the Jacobian struct g2_deserialize returns
+// (z = Montgomery one; all zero for the identity) -- for the items that decode; undecodable items leave their struct untouched
+// (blsSignatureDeserialize, hbls.cu).  out may then be null.
+__global__ void k_g2_decode_pair(size_t n, const uint8_t* in, g2a* out, uint8_t* ok, int check_order, g2* out_jac = nullptr) {
     const size_t i = HB_TID >> 1; if (i >= n) return;                    // a pair leaves together
     g2 p; bool good = g2_deserialize(p, in + 96 * i, false);
     if (good && check_order && !pt_is_inf(p)) {
@@ -361,10 +364,21 @@ __global__ void k_g2_decode_pair(size_t n, const uint8_t* in, g2a* out, uint8_t*
         good = g2_in_subgroup(q);
     }
     if ((threadIdx.x & 1) == 0) {
-        g2a a;
-        if (!good || pt_is_inf(p)) { fp2_zero(a.x); fp2_zero(a.y); } else { a.x = p.x; a.y = p.y; }
-        out[i] = a; ok[i] = good ? 1 : 0;
+        if (out) {
+            g2a a;
+            if (!good || pt_is_inf(p)) { fp2_zero(a.x); fp2_zero(a.y); } else { a.x = p.x; a.y = p.y; }
+            out[i] = a;
+        }
+        if (out_jac && good) out_jac[i] = p;
+        ok[i] = good ? 1 : 0;
     }
+}
+// per-item H(m) of a coalesced batch (hbls.cu): item i takes the point of its distinct message idx[i]; the host hashed each distinct
+// message once (or found it in the H(m) cache)
+__global__ void k_hm_gather(size_t n, const uint32_t* idx, const g2a* dist_hm, const uint8_t* dist_ok, g2a* hm, uint8_t* ok) {
+    const size_t i = HB_TID; if (i >= n) return;
+    const uint32_t d = idx[i];
+    hm[i] = dist_hm[d]; ok[i] = dist_ok[d];
 }
 __global__ void k_hash_to_g2_pair(size_t n, const uint8_t* msgs, uint32_t msg_len, g2a* out, uint8_t* ok) {
     const size_t i = HB_TID >> 1; if (i >= n) return;
@@ -1162,7 +1176,8 @@ __global__ void k_sign_hm_gls_pair(size_t n, const uint64_t* digits, const g2a* 
 }
 
 // ---- single-element ops behind the herumi-shaped C ABI (one thread; latency is launch-bound)
-enum { OP_G1_ADD = 1, OP_G1_SUB, OP_G2_ADD, OP_G1_EQ, OP_G2_EQ, OP_G1_SER, OP_G2_SER, OP_G1_DES, OP_G2_DES, OP_MAP_SER, OP_G2_DES_ADD };
+// (Sign / PublicKey Deserialize run batched: k_g2_decode_pair with the struct epilogue, k_g1_decode_jac)
+enum { OP_G1_ADD = 1, OP_G1_SUB, OP_G2_ADD, OP_G1_EQ, OP_G2_EQ, OP_G1_SER, OP_G2_SER, OP_MAP_SER, OP_G2_DES_ADD };
 __global__ void k_single(int op, const void* a, const void* b, void* out, int* rc, uint32_t len) {
     if (HB_TID != 0) return;
     switch (op) {
@@ -1174,8 +1189,6 @@ __global__ void k_single(int op, const void* a, const void* b, void* out, int* r
     case OP_G2_EQ: { g2 x = *(const g2*)a, y = *(const g2*)b; *rc = pt_eq(x, y) ? 1 : 0; break; }
     case OP_G1_SER: { g1 x = *(const g1*)a; g1_serialize((uint8_t*)out, x); *rc = 48; break; }
     case OP_G2_SER: { g2 x = *(const g2*)a; g2_serialize((uint8_t*)out, x); *rc = 96; break; }
-    case OP_G1_DES: { g1 x; bool g = g1_deserialize(x, (const uint8_t*)a, true); if (g) *(g1*)out = x; *rc = g ? 48 : 0; break; }
-    case OP_G2_DES: { g2 x; bool g = g2_deserialize(x, (const uint8_t*)a, true); if (g) *(g2*)out = x; *rc = g ? 96 : 0; break; }
     case OP_MAP_SER: { g2 h; bool g = map_to_g2(h, (const uint8_t*)a, len); if (g) g2_serialize((uint8_t*)out, h); *rc = g ? 0 : -1; break; }
     case OP_G2_DES_ADD: {   // ballot box: out (Jacobian running sum) += decode(a); rc = 96 ok / 0 undecodable (sum untouched)
         g2 x; bool g = g2_deserialize(x, (const uint8_t*)a, true);

@@ -11,9 +11,15 @@
  *     internal/chain/engine.go:619-642 verifySignature, consensus/leader.go:227-290 onCommit loop).
  *
  * Conventions: plain pointers and sizes only; all memory caller-owned; no callbacks; int error codes.
- * Threading: every function may be called from any thread after blsInit; calls are serialised by one library mutex and
- * (except hbls_aggregate_verify_batch_device on a caller stream) one library stream.  Scratch memory is per stream, so
- * asynchronous device-pointer calls on DIFFERENT streams do not share intermediates; calls on one stream are stream-ordered.
+ * Threading: every function may be called from any thread after blsInit.  Concurrent per-call blsVerifyHash / blsVerify,
+ * blsSignHash / blsSign, blsSignatureDeserialize, blsPublicKeyDeserialize and blsGetPublicKey calls are COALESCED: each queues its
+ * request, and one of the waiting callers (no extra thread) takes the library mutex, drains up to coop_max queued requests and runs
+ * them as one batched device pass per operation kind -- each caller gets exactly the result and output bytes of a lone call.  A
+ * request waits at most for the batch in flight (or the batch call holding the mutex) and then leaves in the next batch; a lone
+ * caller runs a batch of one at once.  Everything else -- Add / Sub / IsEqual / Serialize and the batch entry points of Part 2 --
+ * runs one call at a time under the library mutex.  All of it runs on one library stream (except
+ * hbls_aggregate_verify_batch_device on a caller stream).  Scratch memory is per stream, so asynchronous device-pointer calls on
+ * DIFFERENT streams do not share intermediates; calls on one stream are stream-ordered.
  * Messages: only the first min(len, 48) bytes enter the map to G2 (mcl setArrayMask; SURVEY A.3); batch entry points take the
  * message stride msg_len and read min(msg_len, 48) bytes per item.
  * Identity operands: VerifyHash / aggregate-verify with an identity public key (e.g. an empty bitmap) returns 0 -- a zero key would
@@ -238,6 +244,9 @@ int hbls_get_public_key_batch(size_t k, const uint8_t* sk32, uint8_t* pk48_out);
  * id -- hence the commit payload -- become known).  hbls_set_param("hm_cache", 0) turns the cache off.  0 ok. */
 int hbls_hash_prefetch(const void* msg, size_t msg_len);
 int hbls_hash_cache_stats(uint64_t* hits, uint64_t* misses);
+/* coalescing of the per-call operations (Threading above), counted since load: requests queued, batches run, largest batch.
+ * requests == batches when every call ran alone.  Any pointer may be NULL.  0 ok. */
+int hbls_coalesce_stats(uint64_t* requests, uint64_t* batches, uint64_t* largest_batch);
 
 /* ------------------------------------------------------------------ probes used by tests / bench */
 /* message -> G2 point, serialized (the H(m) of SignHash/VerifyHash): 0 ok, -1 undefined */
