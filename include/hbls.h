@@ -143,7 +143,11 @@ int hbls_last_batch_info(hbls_batch_info* out);
 /* tuning knobs (tests, sweeps): "rlc_min" (rounds from which mode 1 batches in groups), "rlc_g" (0 auto / 4 / 8), "coop_max" (exact
  * checks of at most this many rounds use the warp-per-round latency kernel, 0 = never), "tpsm" (resident threads per SM of the
  * thread-per-item kernels), "tpsm_split" (lane-pair kernels), "tpsm_light", "coop_wpsm" (resident warps per SM of the warp-per-round kernels), "hm_cache" (0: H(m) cache off), "hash_coop_max" (hash-to-G2 of at most this many messages runs one warp per message), "mask_sort" (1: large batches aggregate keys in the order of the rounds' addition counts), "hash_split" (large batches hash in 0: one kernel, 1: map + cofactor clearing, 2: map + cofactor clearing + affine conversion), "rlc_two_phase" (batched pairing as 0: one kernel, 1: two kernels when the batch fills the chip, 2: always two kernels), "hash_fallback" (test hook: 1 forces the warp-per-message hash through its complete-formula fall-back), "tpsm_sw" (resident threads per SM of the map kernel), "overlap" (1: small batches decode signatures and
- * hash messages on two auxiliary streams beside the key aggregation).  Defaults come from HBLS_RLC_MIN, HBLS_RLC_G, HBLS_COOP_MAX,
+ * hash messages on two auxiliary streams beside the key aggregation), "scale_split" (batched groups scale keys and signatures in 0: one
+ * kernel, 1: a G1 kernel and a G2 kernel), "decode_split" (large batches decode signatures in 0: one kernel with the subgroup test,
+ * 1: decode + a separate subgroup kernel), "exact_two_phase" (1: exact checks beyond coop_max and the exact pass over failed groups run
+ * as line kernel + accumulator kernel when rlc_two_phase is 2), "tpsm_cof", "tpsm_dec", "tpsm_scale", "tpsm_scale_g1", "tpsm_lines",
+ * "tpsm_accum" (resident threads per SM of the cofactor, decode, scaling, line and accumulator kernels).  Defaults come from HBLS_RLC_MIN, HBLS_RLC_G, HBLS_COOP_MAX,
  * HBLS_TPSM, HBLS_TPSM_SPLIT, HBLS_TPSM_LIGHT at blsInit.  0 ok, HBLS_ERR_ARG for an unknown name / bad value. */
 int hbls_set_param(const char* name, long long value);
 long long hbls_get_param(const char* name);

@@ -421,8 +421,9 @@ def _bench_committee(gbls):
     return sks, pks, gbls.Committee(pks)
 
 def test_headline_configuration_rejects_bad_rounds(gbls, oracle):
-    """The benchmark's own configuration -- B = 303 104 rounds = 37 888 strided groups of 8, k_rlc_pairing_split<8> in 512-thread
-    lock-stepped persistent CTAs -- with >= 30 seeded bad rounds of five kinds.  Per-round booleans equal the oracle's on every
+    """The benchmark's own configuration -- B = 303 104 rounds = 37 888 strided groups of 8 (one chunk of the two-kernel pairing
+    k_rlc_lines_split<8> / k_rlc_accum_split<8> in 512-thread lock-stepped persistent CTAs; the fused k_rlc_pairing_split<8> only runs
+    with rlc_two_phase 0, see tests/test_gpu_paths.py) -- with >= 30 seeded bad rounds of seven kinds.  Per-round booleans equal the oracle's on every
     bad round and on a 2 000-round random sample; hbls_last_batch_info shows that the G = 8 kernel itself rejected exactly the
     groups that hold a bad round, and that only their rounds went through the exact pass."""
     import bench
@@ -770,9 +771,9 @@ def test_hash_cache_sign_then_verify(gbls, oracle):
         gbls.SetParam("hm_cache", old)
 
 def test_hash_paths_agree(gbls, oracle):
-    """hash-to-G2 has four device forms: thread per item (large batches; one kernel or map + cofactor kernels), lane pair per item,
-    warp per message with the cofactor clearing on the VM, and that kernel's fall-back for degenerate group-law cases (forced here).
-    All give the oracle's bytes through SignHash, and the same verdicts through a 40-round batch."""
+    """The small-batch hash-to-G2 forms: lane pair per item, warp per message with the cofactor clearing on the VM, and that kernel's
+    fall-back for degenerate group-law cases (forced here).  All give the oracle's bytes through SignHash, and the same verdicts through
+    a 40-round batch.  The thread-per-item forms of large batches (hash_split 0 / 1 / 2) are run by tests/test_gpu_paths.py."""
     n = 8
     sks = [wl.seeded_sk("hp", i) for i in range(n)]
     pks_blob = gbls.GetPublicKeyBatch(b"".join(wl.sk_bytes(k) for k in sks))
